@@ -63,7 +63,15 @@ def parse():
                     help="weak: --rays per GPU; strong: --rays in total, split over the GPUs (BASELINE configs[3,4])")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from Python instead of replaying "
                     "the captured CUDA graphs of the step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (rendered outputs, loss, "
+                         "updated parameters) as DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the B200 arm (--impl ours)")
+    return args
 
 
 # ----------------------------------------------------------------------------- losses (host glue)
@@ -221,12 +229,13 @@ class Trainer:
         torch.cuda.synchronize()
         from emernerf_b200 import _lib
 
-        self.graph_launches = {}
+        self.graph_launches, self.static_out = {}, {}
         for prg in (False, True):
             g = torch.cuda.CUDAGraph()
             n0 = _lib.LAUNCHES
             with torch.cuda.graph(g):
                 self.static_loss[prg] = self._step_body(self.static, prg)
+            self.static_out[prg] = self.body_out
             self.graph_launches[prg] = _lib.LAUNCHES - n0      # library kernels inside this graph
             self.graphs[prg] = g
 
@@ -288,12 +297,15 @@ class Trainer:
                 v.copy_(src[k], non_blocking=True)
             self.graphs[prg].replay()
             self.replayed_launches = getattr(self, "replayed_launches", 0) + self.graph_launches[prg]
-            return self.static_loss[prg]
+            self.last_loss, self.last_out = self.static_loss[prg], self.static_out[prg]
+            return self.last_loss
         if from_host:
             batch = {k: v.to(self.device, non_blocking=True) for k, v in self.host[i % 8].items()}
         else:
             batch = self.dev[i % 8]
-        return self._step_body(batch, prg)
+        self.last_loss = self._step_body(batch, prg)
+        self.last_out = self.body_out
+        return self.last_loss
 
     def _step_body(self, batch, prg):
         from emernerf_b200.radiance_fields.render_utils import render_rays
@@ -310,6 +322,7 @@ class Trainer:
         self.opt.zero_grad()
         (loss * 1024.0).backward()                # GradScaler(2**10).scale(loss), never unscaled (Q17)
         self.sync_and_step(self.opt, self.params)
+        self.body_out = out                       # what render_rays returned: --dump-outputs writes it
         return loss
 
 
@@ -332,6 +345,57 @@ def timed(trainer, steps, from_host, sync):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = t.item()
     return ms
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(trainer, out_dir):
+    """Write what the last timed step computed as ``out_dir/<name>.npy``: every tensor ``render_rays`` returned
+    (``extras.<key>`` for the per-sample extras), the loss, and every field / proposal parameter after the step's
+    Adam update.  Floating arrays are written as float32 (float64 stays float64), others as float64.  Arrays larger
+    than a sample size are flattened and sampled at positions drawn from a generator seeded with 0; the sample size
+    starts at 2^20 elements and halves until the whole dump fits in DUMP_LIMIT_BYTES.  Both depend only on the shapes,
+    so two builds run with the same arguments write the same positions.  Nothing is written unless all of it fits."""
+    import numpy as np
+
+    arrays = {"loss": trainer.last_loss}
+
+    def add(prefix, d):
+        for k, v in d.items():
+            if isinstance(v, dict):
+                add(f"{prefix}{k}.", v)
+            elif torch.is_tensor(v):
+                arrays[prefix + k] = v
+            else:
+                raise SystemExit(f"--dump-outputs: render output {prefix}{k} is a {type(v).__name__}, not a tensor")
+
+    add("", trainer.last_out)
+    arrays.update({f"field.{k}": v for k, v in trainer.field.named_parameters()})
+    for i, p in enumerate(trainer.props):
+        arrays.update({f"prop{i}.{k}": v for k, v in p.named_parameters()})
+
+    def nbytes(t, cap):
+        return min(t.numel(), cap) * (8 if t.dtype == torch.float64 or not t.is_floating_point() else 4)
+
+    cap = 1 << 20
+    while cap > 1 and sum(nbytes(t, cap) for t in arrays.values()) > DUMP_LIMIT_BYTES:
+        cap //= 2
+    torch.cuda.synchronize()
+    out = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > cap:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        a = t.cpu().numpy()
+        out[name] = a.astype(a.dtype if a.dtype == np.float64 else np.float32 if t.is_floating_point() else np.float64)
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_LIMIT_BYTES, total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    return {"dir": out_dir, "arrays": len(out), "bytes": total, "sample_elements": cap}
 
 
 def _safe(fn, *a):
@@ -403,6 +467,9 @@ def run_ours(args):
     torch.cuda.set_device(local)
     device = torch.device("cuda", local)
     if world > 1:
+        if args.dump_outputs:
+            # the sharded optimizer leaves each rank's copy of the parameters partly stale until the next step
+            raise SystemExit("--dump-outputs needs a one-GPU run")
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=device)
 
@@ -427,6 +494,7 @@ def run_ours(args):
     tr.replayed_launches = 0
     ms = timed(tr, args.steps, False, sync)
     launches = (_lib.LAUNCHES - launches0) + tr.replayed_launches
+    dumped = dump_outputs(tr, args.dump_outputs) if args.dump_outputs else None
 
     e2e = None
     if not args.no_e2e:
@@ -615,6 +683,8 @@ def run_ours(args):
     }
     if e2e is not None:
         line["e2e"] = e2e
+    if dumped is not None:
+        line["dumped_outputs"] = dumped
     if full is not None:
         line["full_step"] = full
     if not args.no_cpu_baseline and world == 1:
@@ -760,9 +830,8 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", 0))
     if rank != 0:
         return
-    # every step is a bounded sample (--cpu-rays rays) of the workload; at most 16 of them are timed so that the
-    # arm ends within a few minutes whatever K the caller asks for -- "steps" reports what was actually timed
-    steps, warmup = max(1, min(args.steps, 16)), max(1, min(args.warmup, 2))
+    # every step is a bounded sample (--cpu-rays rays) of the workload
+    steps, warmup = args.steps, max(1, min(args.warmup, 2))
     cb = cpu_baseline(args, steps=steps, warmup=warmup)
     line = {
         "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,

@@ -67,3 +67,49 @@ def assert_close_dict(got, want, tol, path="", skip=()):
         t = tol[k] if isinstance(tol, dict) and k in tol else (tol["*"] if isinstance(tol, dict) else tol)
         e = rel_err(got[k], want[k])
         assert e <= t, f"{path}{k}: rel err {e:.3e} > {t:.1e}"
+
+
+# ---- sampled fixtures: a fixed, seeded sample of every array, so that a whole set of outputs stays a few kB
+SAMPLE = 128
+
+
+def sample_positions(n: int, k: int = SAMPLE) -> torch.Tensor:
+    """Flat positions compared in an array of ``n`` elements: all of them, or ``k`` drawn with seed 0 (sorted)."""
+    if n <= k:
+        return torch.arange(n)
+    return torch.randperm(n, generator=torch.Generator().manual_seed(0))[:k].sort().values
+
+
+def pack_sampled(arrays, k: int = SAMPLE):
+    """{name: tensor} -> the npz entries of one sampled set: ``meta`` (JSON: name -> shape, in order), ``values`` (the
+    sampled elements, concatenated, float32) and ``maxabs`` (each array's full max |x|, the comparison's scale)."""
+    import json
+
+    names = sorted(arrays)
+    vals, scale = [], []
+    for n in names:
+        a = arrays[n].detach().double().cpu().reshape(-1)
+        vals.append(a[sample_positions(a.numel(), k)])
+        scale.append(a.abs().max().item() if a.numel() else 0.0)
+    meta = json.dumps({n: list(arrays[n].shape) for n in names})
+    return {"meta": np.array(meta), "values": (torch.cat(vals) if vals else torch.zeros(0)).float().numpy(),
+            "maxabs": np.array(scale, dtype=np.float64)}
+
+
+def sampled_errors(got, z, prefix: str, k: int = SAMPLE):
+    """Max relative error of each array of ``got`` against the sampled set ``prefix`` of the npz ``z``: the names
+    and shapes must agree; the error is max |got - want| over the sampled positions over the full max |want|."""
+    import json
+
+    meta = json.loads(str(z[prefix + "meta"]))
+    assert sorted(got) == list(meta), (prefix, sorted(set(got) ^ set(meta)))
+    values, maxabs = torch.from_numpy(z[prefix + "values"]).double(), z[prefix + "maxabs"]
+    errs, off = {}, 0
+    for i, n in enumerate(meta):
+        a = got[n].detach().double().cpu()
+        assert list(a.shape) == meta[n], (prefix + n, list(a.shape), meta[n])
+        pos = sample_positions(a.numel(), k)
+        want = values[off:off + len(pos)]
+        off += len(pos)
+        errs[n] = ((a.reshape(-1)[pos] - want).abs().max().item() / max(maxabs[i], 1e-12)) if len(pos) else 0.0
+    return errs

@@ -1,28 +1,28 @@
-"""The drop-in claim, end to end, at the REAL configuration (build container only).
+"""The drop-in at the REAL configuration, against vectors the reference's own code produced.
 
-The reference's own ``builders.py`` (unmodified, imported from /root/reference) builds the model and the
-proposal estimator from the reference's own ``configs/default_config.yaml`` twice:
+``python tests/live_dropin_builders.py`` (needs the reference checkout, EMER_REFERENCE_ROOT) writes two fixtures:
 
-  ref   <file>   with the reference's classes (oracle stand-ins for tiny-cuda-nn / nerfacc)
-                 -> saves the state-dicts, a ray batch and the rendered outputs
-  ours  <file>   after ``emernerf_b200.install_dropin()`` (C ABI answered by tests/cabi_emulator.py)
-                 -> loads them, renders the same rays through the reference's import names, prints the errors
+  builders.npz  the reference's unmodified ``builders.py`` builds the model and the proposal estimator from its
+                ``configs/default_config.yaml`` with every branch switched on (dynamic, flow, shadow, feature head; real
+                table sizes, 203 MB of grids) and the reference's classes (oracle stand-ins for tiny-cuda-nn / nerfacc);
+                stored: the state-dict's names and shapes, the parameter count and a sample of the rendered outputs
+  raygen.npz    the reference's ``get_rays`` (datasets/base/pixel_source.py, executed from its source file) on seeded
+                pixels and poses, every element
 
-Only ``omegaconf`` (annotation only) and ``datasets.base`` (annotation only; its real import chain needs timm) are
-stubbed.  The configuration is default_config.yaml with every branch switched on (dynamic, flow, shadow, feature
-head) so that every config key the builders read is exercised; table sizes are the real ones (203 MB of grids).
+tests/test_live_reference_variants.py builds the same model with ``emernerf_b200.configs`` (same seed, hence the same
+weights) and compares.  Only ``omegaconf`` (annotation only) and ``datasets.base`` (annotation only; its real import
+chain needs timm) are stubbed while the reference builds.
 """
 from __future__ import annotations
 
-import json
 import os
 import re
 import sys
 import types
 import warnings
 
+import numpy as np
 import torch
-import yaml
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
@@ -33,6 +33,7 @@ for p in (ROOT, HERE, os.path.join(HERE, "golden")):
 warnings.filterwarnings("ignore")
 
 N_RAYS, T = 40, 12
+AABB = [-25.0, -35.0, -2.0, 90.0, 45.0, 25.0]      # the dataset's aabb, which builders.py gives the model
 
 
 class Cfg(dict):
@@ -59,6 +60,8 @@ def to_cfg(o):
 
 
 def load_cfg():
+    import yaml
+
     with open(os.path.join(REF, "configs", "default_config.yaml")) as f:
         cfg = to_cfg(yaml.safe_load(f))
     head = cfg.nerf.model.head
@@ -77,7 +80,7 @@ def dataset_stub():
     px = types.SimpleNamespace(features=None)
     return types.SimpleNamespace(num_train_timesteps=T, test_pixel_set=None, num_img_timesteps=T,
                                  unique_normalized_training_timestamps=torch.linspace(0, 1, T),
-                                 aabb=torch.tensor([-25.0, -35.0, -2.0, 90.0, 45.0, 25.0]), pixel_source=px)
+                                 aabb=torch.tensor(AABB), pixel_source=px)
 
 
 def stub_annotation_only_modules():
@@ -130,52 +133,87 @@ def flatten(d, prefix=""):
     return out
 
 
-def main():
-    mode, path = sys.argv[1], sys.argv[2]
+def randomise_tables(model, props):
+    g = torch.Generator().manual_seed(1)
+    with torch.no_grad():                       # give the scene structure (tcnn's own init is ~1e-4)
+        for m in [model] + props:
+            for k, v in m.named_parameters():
+                if k.endswith("tcnn_encoding.params"):
+                    v.copy_(torch.randn(v.shape, generator=g) * 0.5)
+
+
+def build_ours():
+    """The same model and networks from this package: default_config's values (emernerf_b200.configs, every branch on),
+    the same seed as the reference's build."""
+    from emernerf_b200 import configs
+
+    cfg = configs.make_cfg("flow_feat", num_timesteps=T)
+    model, props, est, _ = configs.build_hot_path(cfg, "cpu")
+    for m in [model] + props:
+        m.set_aabb(AABB)
+    randomise_tables(model, props)
+    return model, est, props, cfg
+
+
+def render_ours():
+    """(model, parameter count, flat outputs) of the drop-in on the fixture's rays."""
+    from emernerf_b200.radiance_fields.render_utils import render_rays
+
+    model, est, props, cfg = build_ours()
+    for m in (model, est, *props):
+        m.eval()
+    with torch.no_grad():
+        out = render_rays(radiance_field=model, proposal_estimator=est, proposal_networks=props,
+                          data_dict=make_batch(), cfg=cfg, proposal_requires_grad=False, return_decomposition=True)
+    return model, sum(p.numel() for p in model.parameters()), flatten(out)
+
+
+RAYGEN_RAYS = 777
+RAYGEN_ALL = 3 * RAYGEN_RAYS          # sample size that keeps every element of every get_rays output
+
+
+def raygen_inputs():
+    g = torch.Generator().manual_seed(0)
+    R = RAYGEN_RAYS
+    x, y = torch.randint(0, 960, (R,), generator=g).float(), torch.randint(0, 640, (R,), generator=g).float()
+    c2w = torch.eye(4).repeat(R, 1, 1) + torch.randn(R, 4, 4, generator=g) * 0.3
+    K = torch.tensor([[1030.0, 0, 480], [0, 1030, 320], [0, 0, 1]]).repeat(R, 1, 1)
+    return x, y, c2w, K
+
+
+def raygen_outputs(get_rays):
+    """get_rays on per-ray poses and on one shared pose: {"batched/<i>", "shared/<i>"} for each returned tensor."""
+    x, y, c2w, K = raygen_inputs()
+    res = {f"batched/{i}": t for i, t in enumerate(get_rays(x, y, c2w, K))}
+    res.update({f"shared/{i}": t for i, t in enumerate(get_rays(x, y, c2w[0], K[0]))})
+    return res
+
+
+def write_golden():
+    from helpers import GOLDEN_DIR, pack_sampled
+    from oracle import ref_shims
+
     cfg = load_cfg()
     stub_annotation_only_modules()
     sys.path.insert(0, REF)
-    if mode == "ref":
-        from oracle import ref_shims
+    ref_shims.install()
+    torch.manual_seed(0)
+    model, est, props = build_with_reference_builders(cfg)
+    randomise_tables(model, props)
+    assert type(model).__module__ == "radiance_fields.radiance_field", type(model).__module__
+    out = flatten(render(model, est, props, make_batch(), cfg))
+    sd = model.state_dict()
+    store = {f"out/{k}": v for k, v in pack_sampled(out).items()}
+    store["state_dict"] = np.array(repr({k: list(v.shape) for k, v in sd.items()}))
+    store["n_params"] = np.array(sum(p.numel() for p in model.parameters()))
+    np.savez_compressed(os.path.join(GOLDEN_DIR, "builders.npz"), **store)
 
-        ref_shims.install()
-        torch.manual_seed(0)
-        model, est, props = build_with_reference_builders(cfg)
-        g = torch.Generator().manual_seed(1)
-        with torch.no_grad():                       # give the scene structure (tcnn's own init is ~1e-4)
-            for m in [model] + props:
-                for k, v in m.named_parameters():
-                    if k.endswith("tcnn_encoding.params"):
-                        v.copy_(torch.randn(v.shape, generator=g) * 0.5)
-        assert type(model).__module__ == "radiance_fields.radiance_field", type(model).__module__
-        batch = make_batch()
-        out = render(model, est, props, dict(batch), cfg)
-        torch.save({"model": model.state_dict(), "props": [p.state_dict() for p in props], "batch": batch,
-                    "out": flatten(out)}, path)
-        print("JSON:" + json.dumps({"keys": sorted(flatten(out)), "n_params": sum(p.numel() for p in model.parameters())}))
-    else:
-        import cabi_emulator
-        import emernerf_b200
-
-        emernerf_b200.install_dropin()
-        cabi_emulator.install(types.SimpleNamespace(setattr=setattr))
-        blob = torch.load(path)
-        model, est, props = build_with_reference_builders(cfg)
-        assert type(model).__module__.startswith("emernerf_b200."), type(model).__module__
-        assert type(est).__module__.startswith("emernerf_b200.") and type(props[0]).__module__.startswith("emernerf_b200.")
-        model.load_state_dict(blob["model"])                       # strict: same keys, same shapes
-        for p, sd in zip(props, blob["props"]):
-            p.load_state_dict(sd)
-        got = flatten(render(model, est, props, dict(blob["batch"]), cfg))
-        want = blob["out"]
-        assert set(got) == set(want), sorted(set(got) ^ set(want))
-        errs = {}
-        for k in want:
-            a, b = got[k].double(), want[k].double()
-            assert a.shape == b.shape, (k, a.shape, b.shape)
-            errs[k] = ((a - b).abs().max() / b.abs().max().clamp_min(1e-12)).item()
-        print("JSON:" + json.dumps({"errors": errs, "calls": sorted(set(cabi_emulator.CALLS))}))
+    src = open(os.path.join(REF, "datasets", "base", "pixel_source.py")).read()
+    body = src[src.index("def get_rays("):src.index("class ScenePixelSource")]
+    ns = {}
+    exec("import torch\nfrom torch import Tensor\nfrom typing import Tuple\n" + body, ns)
+    np.savez_compressed(os.path.join(GOLDEN_DIR, "raygen.npz"), **pack_sampled(raygen_outputs(ns["get_rays"]), k=RAYGEN_ALL))
 
 
 if __name__ == "__main__":
-    main()
+    write_golden()

@@ -1,21 +1,22 @@
-"""Option variants of the field / estimator, REFERENCE vs DROP-IN, live (build container only).
+"""Option variants of the field / estimator beyond the four golden cases (constructor options and data-dict shapes of
+SURVEY.md section 8b that the shipped configs do not exercise).
 
-Run as a script by tests/test_live_reference_variants.py in a subprocess (the reference's module names
-``radiance_fields`` / ``third_party`` go into ``sys.modules``).  For every variant the reference's own classes
-(with the oracle stand-ins for tiny-cuda-nn / nerfacc, oracle/ref_shims.py) and the drop-in's classes (with the
-C ABI answered by tests/cabi_emulator.py) are built with the same constructor arguments, the reference's
-state-dict is loaded into the drop-in, both render the same rays, and the maximum relative error of every
-output is printed as one JSON object.  What this covers beyond the four golden cases: the constructor options
-and data-dict shapes of SURVEY.md section 8b that the shipped configs do not exercise.
+``run_variant(name, side)`` builds one variant from ``side``'s classes (the reference's or the drop-in's: both draw the
+same weights from the same seeds), renders the same rays and returns every output, plus, in training mode, the
+proposal loss and the parameter gradients.  tests/test_live_reference_variants.py runs the drop-in (C ABI answered by
+tests/cabi_emulator.py) against ``tests/golden/variants.npz``, which this script writes from the reference's own
+classes (with the oracle stand-ins for tiny-cuda-nn / nerfacc, oracle/ref_shims.py):
+
+    python tests/live_reference_variants.py        # needs the reference checkout (EMER_REFERENCE_ROOT)
 """
 from __future__ import annotations
 
-import json
 import os
 import sys
 import types
 import warnings
 
+import numpy as np
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -25,35 +26,38 @@ for p in (ROOT, HERE, os.path.join(HERE, "golden")):
         sys.path.insert(0, p)
 warnings.filterwarnings("ignore")
 
-from oracle import ref_shims  # noqa: E402
-
-ref_shims.install()
-
-import cabi_emulator  # noqa: E402
 import cases  # noqa: E402
-from radiance_fields import RadianceField as RefField, build_density_field as ref_build_density  # noqa: E402
-from radiance_fields.encodings import HashEncoder as RefEncoder  # noqa: E402
-from radiance_fields.render_utils import render_rays as ref_render_rays  # noqa: E402
-from third_party.nerfacc_prop_net import PropNetEstimator as RefEstimator  # noqa: E402
 
-from emernerf_b200.radiance_fields import RadianceField, build_density_field  # noqa: E402
-from emernerf_b200.radiance_fields.encodings import HashEncoder  # noqa: E402
-from emernerf_b200.radiance_fields.render_utils import render_rays  # noqa: E402
-from emernerf_b200.third_party.nerfacc_prop_net import PropNetEstimator  # noqa: E402
+GOLDEN = os.path.join(HERE, "golden", "variants.npz")
 
 
-class _Patch:
-    """monkeypatch-like object for cabi_emulator.install outside pytest."""
+def ours():
+    """The drop-in's classes (the C ABI must be answered: a GPU, or tests/cabi_emulator.py)."""
+    from emernerf_b200.radiance_fields import RadianceField, build_density_field
+    from emernerf_b200.radiance_fields.encodings import HashEncoder
+    from emernerf_b200.radiance_fields.render_utils import render_rays
+    from emernerf_b200.third_party.nerfacc_prop_net import PropNetEstimator
 
-    def setattr(self, obj, name, value):
-        setattr(obj, name, value)
+    return types.SimpleNamespace(HashEncoder=HashEncoder, RadianceField=RadianceField,
+                                 build_density_field=build_density_field, render_rays=render_rays,
+                                 PropNetEstimator=PropNetEstimator)
 
 
-cabi_emulator.install(_Patch())
+def reference():
+    """The reference's own classes, unmodified, with the oracle stand-ins for tiny-cuda-nn / nerfacc."""
+    from oracle import ref_shims
 
-REF = types.SimpleNamespace(HashEncoder=RefEncoder, RadianceField=RefField, build_density_field=ref_build_density)
-OURS = types.SimpleNamespace(HashEncoder=HashEncoder, RadianceField=RadianceField,
-                             build_density_field=build_density_field)
+    assert ref_shims.reference_available(), "needs the reference checkout (EMER_REFERENCE_ROOT)"
+    ref_shims.install()
+    from radiance_fields import RadianceField, build_density_field
+    from radiance_fields.encodings import HashEncoder
+    from radiance_fields.render_utils import render_rays
+    from third_party.nerfacc_prop_net import PropNetEstimator
+
+    return types.SimpleNamespace(HashEncoder=HashEncoder, RadianceField=RadianceField,
+                                 build_density_field=build_density_field, render_rays=render_rays,
+                                 PropNetEstimator=PropNetEstimator)
+
 
 BASE = dict(geometry_feature_dim=64, base_mlp_layer_width=64, head_mlp_layer_width=64, enable_cam_embedding=False,
             enable_img_embedding=True, num_cams=cases.N_CAMS, appearance_embedding_dim=16, semantic_feature_dim=64,
@@ -119,29 +123,23 @@ def randomise(field, props, seed=1):
                     v.copy_(torch.randn(v.shape, generator=g) * 0.5)
 
 
-def rel(a, b):
-    a, b = a.detach().double(), b.detach().double()
-    return ((a - b).abs().max() / b.abs().max().clamp_min(1e-12)).item()
-
-
-def compare(got, want, errs, prefix=""):
-    assert set(got) == set(want), (prefix, sorted(set(got) ^ set(want)))
-    for k in want:
-        if isinstance(want[k], dict):
-            compare(got[k], want[k], errs, prefix + k + "/")
+def flatten(d, prefix=""):
+    out = {}
+    for k, v in d.items():
+        if isinstance(v, dict):
+            out.update(flatten(v, prefix + k + "/"))
         else:
-            assert got[k].shape == want[k].shape, (prefix + k, got[k].shape, want[k].shape)
-            errs[prefix + k] = rel(got[k], want[k])
+            out[prefix + k] = v
+    return out
 
 
-def run_variant(name):
+def run_variant(name, side):
+    """Every output of variant ``name`` rendered with ``side``'s classes, flat: ``out/<key>``, and in training mode
+    ``prop_loss`` and ``grad/<parameter>`` / ``grad/prop<i>/<parameter>`` for every parameter that receives a gradient.
+    A refusal (the same on both sides is parity too) is returned as ``{"raises": "<type>: <message>"}``."""
     kwargs, dynamic, flow, edit, cfg_edit, est_kw, mode = VARIANTS[name]
-    rf, rp = build(REF, kwargs, dynamic, flow)
-    randomise(rf, rp)
-    of, op = build(OURS, kwargs, dynamic, flow)
-    of.load_state_dict(rf.state_dict())
-    for a, b in zip(op, rp):
-        a.load_state_dict(b.state_dict())
+    field, props = build(side, kwargs, dynamic, flow)
+    randomise(field, props)
     case = "flow_feat" if edit in ("features", "features384") else "static"
     batch = cases.make_batch(case)
     if edit == "features384":
@@ -160,74 +158,50 @@ def run_variant(name):
     for k, v in cfg_edit.items():
         setattr(cfg.nerf.propnet, k, v)
     if n_props is not None:
-        # the same networks on both sides: drop one, or append a third built like the second
-        if n_props < len(rp):
-            rp, op = rp[:n_props], op[:n_props]
-        while len(rp) < n_props:
+        # drop one network, or append a third built like the second
+        props = props[:n_props]
+        while len(props) < n_props:
             e = cases.ENC_PROP[-1]
-            extra = []
-            for ns in (REF, OURS):
-                torch.manual_seed(9)
-                p = ns.build_density_field(n_input_dims=3, n_levels=e["n_levels"], max_resolution=e["max_resolution"],
-                                           log2_hashmap_size=e["log2_hashmap_size"],
-                                           n_features_per_level=e["n_features_per_level"], unbounded=True)
-                p.set_aabb(cases.AABB)
-                extra.append(p)
-            randomise(extra[0], [], seed=3)
-            extra[1].load_state_dict(extra[0].state_dict())
-            rp, op = rp + [extra[0]], op + [extra[1]]
+            torch.manual_seed(9)
+            p = side.build_density_field(n_input_dims=3, n_levels=e["n_levels"], max_resolution=e["max_resolution"],
+                                         log2_hashmap_size=e["log2_hashmap_size"],
+                                         n_features_per_level=e["n_features_per_level"], unbounded=True)
+            p.set_aabb(cases.AABB)
+            randomise(p, [], seed=3)
+            props.append(p)
     train = mode == "train"
-    r_est = RefEstimator(torch.optim.Adam([q for p in rp for q in p.parameters()], lr=0.01), None, **est_kw)
-    o_est = PropNetEstimator(torch.optim.Adam([q for p in op for q in p.parameters()], lr=0.01), None, **est_kw)
-    for m in (rf, of, r_est, o_est, *rp, *op):
+    est = side.PropNetEstimator(torch.optim.Adam([q for p in props for q in p.parameters()], lr=0.01), None, **est_kw)
+    for m in (field, est, *props):
         m.train(train)
-    errs = {}
-    failures = []
     with torch.set_grad_enabled(train):
-        for fn, args in ((ref_render_rays, (rf, r_est, rp)), (render_rays, (of, o_est, op))):
-            torch.manual_seed(77)
-            try:
-                failures.append(None)
-                res = fn(*args, dict(batch), cfg, proposal_requires_grad=train, return_decomposition=not train)
-            except (AssertionError, ValueError, KeyError) as e:          # same refusal on both sides is parity too
-                failures[-1] = (type(e).__name__, str(e))
-                res = None
-            if fn is ref_render_rays:
-                want = res
-            else:
-                got = res
-    if failures[0] is not None or failures[1] is not None:
-        assert failures[0] == failures[1], failures
-        return {"raises:" + failures[0][0]: 0.0}
-    compare(got, want, errs)
+        torch.manual_seed(77)
+        try:
+            out = side.render_rays(field, est, props, dict(batch), cfg, proposal_requires_grad=train,
+                                   return_decomposition=not train)
+        except (AssertionError, ValueError, KeyError) as e:
+            return {"raises": f"{type(e).__name__}: {e}"}
+    res = flatten(out, "out/")
     if train:
-        wl = r_est.compute_loss(want["extras"]["trans"], 1024.0)
-        gl = o_est.compute_loss(got["extras"]["trans"], 1024.0)
-        errs["prop_loss"] = abs(gl.item() - wl.item()) / max(1.0, abs(wl.item()))
-        loss_w = (want["rgb"] - batch["pixels"]).square().mean() + want["depth"].mean() * 1e-2
-        loss_g = (got["rgb"] - batch["pixels"]).square().mean() + got["depth"].mean() * 1e-2
-        (loss_w + wl).backward()
-        (loss_g + gl).backward()
-        ref_grads = dict(rf.named_parameters())
-        for k, v in of.named_parameters():
-            w = ref_grads[k].grad
-            assert (v.grad is None) == (w is None), k
-            if w is not None:
-                errs["grad/" + k] = rel(v.grad, w)
-        for i, (a, b) in enumerate(zip(op, rp)):
-            rg = dict(b.named_parameters())
-            for k, v in a.named_parameters():
-                w = rg[k].grad
-                assert (v.grad is None) == (w is None), (i, k)
-                if w is not None:
-                    errs[f"grad/prop{i}/" + k] = rel(v.grad, w)
-    return errs
+        ploss = est.compute_loss(out["extras"]["trans"], 1024.0)
+        res["prop_loss"] = ploss
+        loss = (out["rgb"] - batch["pixels"]).square().mean() + out["depth"].mean() * 1e-2
+        (loss + ploss).backward()
+        res.update({"grad/" + k: v.grad for k, v in field.named_parameters() if v.grad is not None})
+        for i, p in enumerate(props):
+            res.update({f"grad/prop{i}/" + k: v.grad for k, v in p.named_parameters() if v.grad is not None})
+    return {k: v if isinstance(v, str) else v.detach() for k, v in res.items()}
 
 
 if __name__ == "__main__":
-    assert ref_shims.reference_available(), "needs /root/reference"
-    out = {}
-    for name in (sys.argv[1:] or list(VARIANTS)):
-        del cabi_emulator.CALLS[:]
-        out[name] = {"errors": run_variant(name), "calls": sorted(set(cabi_emulator.CALLS))}
-    print("JSON:" + json.dumps(out))
+    from helpers import pack_sampled
+
+    ref = reference()
+    store = {}
+    for name in VARIANTS:
+        res = run_variant(name, ref)
+        if "raises" in res:
+            store[f"{name}/raises"] = np.array(res["raises"])
+        else:
+            store.update({f"{name}/{k}": v for k, v in pack_sampled(res).items()})
+    np.savez_compressed(GOLDEN, **store)
+    print(GOLDEN, os.path.getsize(GOLDEN), "bytes")

@@ -1,6 +1,5 @@
 """The functional oracle against the committed golden vectors (generated from the reference's
-own Python by tests/golden/make_golden.py), plus -- in the build container only -- a live
-re-run of the reference to prove the fixtures are reproducible."""
+own Python by tests/golden/make_golden.py)."""
 import pytest
 import torch
 
@@ -82,18 +81,3 @@ def test_oracle_matches_golden_gradients(case):
     for k, gr in zip(sorted(wantp), gotp):
         assert rel_err(gr, wantp[k]) < 1e-4, k
 
-
-@pytest.mark.reference
-def test_fixtures_reproducible_from_reference(tmp_path):
-    """Re-run the reference itself (build container only) and compare with the committed fixture."""
-    import subprocess, sys, os, shutil, numpy as np
-    here = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-    work = tmp_path / "golden"
-    shutil.copytree(here, work, ignore=shutil.ignore_patterns("*.npz", "__pycache__"))
-    env = dict(os.environ, PYTHONPATH=os.path.dirname(os.path.dirname(here)))
-    subprocess.run([sys.executable, str(work / "make_golden.py"), "static"], check=True, env=env,
-                   cwd=os.path.dirname(os.path.dirname(here)), capture_output=True)
-    a, b = np.load(work / "static.npz"), np.load(os.path.join(here, "static.npz"))
-    assert set(a.files) == set(b.files)
-    for k in a.files:
-        assert np.allclose(a[k], b[k], rtol=1e-6, atol=1e-7), k
